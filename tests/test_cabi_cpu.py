@@ -45,8 +45,10 @@ def test_plugin_abi_symbols_exported():
     assert hasattr(lib, "_polars_plugin_get_last_error_message")
 
 
-@pytest.mark.skipif(os.path.exists("/dev/nvidia0"), reason="needs a machine without a GPU")
 def test_no_gpu_fails_loudly_no_cpu_fallback():
+    import torch
+    if torch.cuda.device_count():      # any visible device, whatever its /dev node is called
+        pytest.skip("needs a machine without a GPU")
     import polars_b200 as plb
     with pytest.raises(plb.B200Error) as e:
         plb.elementwise("add", np.arange(4), np.arange(4))
